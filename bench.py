@@ -26,6 +26,9 @@ rank, every rank searches ALL queries of the step on its shard, the tiles are al
 (distance, global id) on the GPU inside the timed region.
 
 `--impl reference` times the CPU restatement of the reference (oracle/, all host threads) on the same index image.
+`--dump-outputs DIR` writes what the last timed step returned (ids, distances, counts) as .npy files.  Data and queries
+are seeded and the index image comes from the --cache directory once built (the GPU builder's graph depends on thread
+interleaving), so two builds of the project run against the same cache can be compared output for output.
 """
 import argparse
 import hashlib
@@ -94,7 +97,12 @@ def parse_args():
     ap.add_argument("--cache", default=os.environ.get("GRANNE_B200_BENCH_CACHE", "/dev/shm/granne_b200_bench_cache"),
                     help="directory for the index file image shared by all runs on this box ('' = no cache)")
     ap.add_argument("--no-fallback", action="store_true", help="fail instead of retrying with 10x fewer elements")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (float32 / float64), so that "
+                         "two builds can be compared output for output on the same seeded inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be >= 1")
     kind, n, dim, mode, base = CONFIGS[a.config]
     a.kind = a.kind or kind
     a.n = a.n or n
@@ -353,6 +361,26 @@ def build_or_load_index(torch, granne_b200, a, dev, container, seed):
             "write_index_s": write_s}
     cache_store(path, data, prov)
     return index, data, prov
+
+
+DUMP_LIMIT = 64 << 20    # bytes written by --dump-outputs at most
+
+
+def dump_outputs(directory, arrays, limit=DUMP_LIMIT):
+    """Writes `arrays` (one row per query; ids as u32 bits or i64, distances, counts) as DIR/<name>.npy: float32 stays
+    float32, every integer type becomes float64 (exact for ids below 2^53).  When they would exceed `limit` bytes, a
+    fixed seeded sample of the rows is written instead, with the sampled row numbers as rows.npy."""
+    out = {name: v if v.dtype == np.float32 else v.astype(np.float64) for name, v in arrays.items()}
+    nrows = next(iter(out.values())).shape[0]
+    total = sum(v.nbytes for v in out.values())
+    if total > limit:
+        keep = int(nrows * limit // (total + 8 * nrows))
+        rows = np.sort(np.random.default_rng(0).choice(nrows, size=keep, replace=False))
+        out = {name: v[rows] for name, v in out.items()}
+        out["rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(v))
 
 
 def workload_config(a, impl, n_used, world, prov=None):
@@ -616,8 +644,10 @@ def run_reference(a):
     t0 = time.time()
     for s in range(a.steps):
         off = (s * 4099) % (queries.shape[0] - per_step + 1)
-        search(queries[off:off + per_step])
+        last = search(queries[off:off + per_step])
     dt = time.time() - t0
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, dict(zip(("ids", "distances", "counts"), last)))
     qps = a.steps * per_step / dt
     prov = shards[0][3]
     line = {"metric": metric_name(a, n), "value": qps, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
@@ -886,6 +916,21 @@ def main():
         ms = float(t.item())
     job_queries = a.steps * a.nq * (1 if partitioned else world)
     value = job_queries / (ms / 1e3)
+    last = None
+    if a.dump_outputs and rank == 0:  # copied now: the solo launches below reuse outs[0]
+        slot = (a.warmup + a.steps - 1) % len(streams)
+        if fused is not None:
+            last = {"ids": fused.ids(slot), "distances": fused.dists(slot)}
+        elif partitioned:
+            last = {"ids": merged[slot][0], "distances": merged[slot][1]}
+        elif world > 1:
+            g = gathered[slot].view(world, 2, a.nq, a.k)
+            last = {"ids": g[:, 0].reshape(-1, a.k), "distances": g[:, 1].reshape(-1, a.k).view(torch.float32)}
+        else:
+            last = {"ids": outs[slot][0], "distances": outs[slot][1], "counts": outs[slot][2]}
+        last = {name: t.cpu().numpy() for name, t in last.items()}
+        if last["ids"].dtype == np.int32:
+            last["ids"] = last["ids"].view(np.uint32)
 
     # kernel-alone duration (single stream, one launch at a time) for the per-launch roofline
     solo = []
@@ -1043,6 +1088,8 @@ def main():
         "multi_gpu_gather": None if world == 1 else ("nccl all_gather + merge_topk_kernel" if partitioned else (
             "p2p peer stores fused into the search kernels" if fused is not None else "nccl all_gather")),
     }
+    if last is not None:
+        dump_outputs(a.dump_outputs, last)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

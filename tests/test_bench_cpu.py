@@ -74,6 +74,30 @@ def test_pack_le_and_sum_container_images(bench, monkeypatch, oracle):
     assert np.array_equal(q, c.queries(32, 4321))  # seeded: both arms see the same queries
 
 
+def test_dump_outputs_types_and_size_cap(bench, monkeypatch, tmp_path):
+    a = _args(bench, monkeypatch, "--config", "c2", "--steps", "3", "--dump-outputs", str(tmp_path / "out"))
+    assert a.steps == 3 and a.dump_outputs == str(tmp_path / "out")
+    with pytest.raises(SystemExit):
+        _args(bench, monkeypatch, "--steps", "0")
+    rng = np.random.default_rng(1)
+    ids = rng.integers(0, 1 << 32, size=(1000, 10), dtype=np.uint64).astype(np.uint32)
+    ids[0, -1] = 0xFFFFFFFF
+    dists = rng.random((1000, 10), dtype=np.float32)
+    counts = np.full(1000, 10, dtype=np.int32)
+    bench.dump_outputs(a.dump_outputs, {"ids": ids, "distances": dists, "counts": counts})
+    got = {n: np.load(tmp_path / "out" / (n + ".npy")) for n in ("ids", "distances", "counts")}
+    assert got["ids"].dtype == np.float64 and np.array_equal(got["ids"], ids.astype(np.float64))
+    assert got["distances"].dtype == np.float32 and np.array_equal(got["distances"], dists)
+    assert got["counts"].dtype == np.float64 and not (tmp_path / "out" / "rows.npy").exists()
+    # above the cap: the same seeded sample of rows every time, row numbers alongside
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"ids": ids, "distances": dists}, limit=40_000)
+    rows = np.load(tmp_path / "a" / "rows.npy").astype(np.int64)
+    assert sum((tmp_path / "a" / f).stat().st_size - 128 for f in ("ids.npy", "distances.npy", "rows.npy")) <= 40_000
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy")) and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "ids.npy"), ids[rows].astype(np.float64))
+
+
 def test_numa_and_peak_helpers_do_not_raise(bench):
     assert isinstance(bench.spread_over_all_cores(), str)
     peak, src = bench.measured_peak_gbs()
